@@ -60,6 +60,9 @@ def parse():
     ap.add_argument("--check-oracle", action="store_true",
                     help="N > 1: rank 0 also proves once with the CPU oracle and compares bit for bit (N = 1 always does, as its cpu_baseline)")
     ap.add_argument("--record", default="", help="also append the JSON line to this file (profiles/r02_bench_*.json)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the proof of the last timed step as DIR/a.npy, b.npy, c.npy (see dump_outputs); the inputs "
+                         "depend only on the arguments, so two builds can be compared output for output")
     return ap.parse_args()
 
 
@@ -263,6 +266,8 @@ def run_reference(a):
     finally:
         orc.set_msm_mode(old)
     assert np.array_equal(proof, proof_w), "window-parallel and chunk-parallel CPU proofs differ"
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, proof, cd.nq)
     line = {
         "impl": "reference", "metric": metric_name(a), "value": val, "unit": "proofs/s", "n_gpus": a.gpus, "steps": a.steps,
         "warmup": a.warmup, "ms_per_step": 1e3 * dt / a.steps, "higher_is_better": True, "scaling": "strong",
@@ -280,6 +285,16 @@ def run_reference(a):
         "gpu_launches": 0,
     }
     emit(a, line)
+
+
+def dump_outputs(d, proof, nq):
+    """What a caller of g16_prove receives -- A (G1), B (G2), C (G1) as affine coordinates of nq Montgomery u64 limbs each --
+    as float64 arrays a (2, 2*nq), b (4, 2*nq), c (2, 2*nq): one row per coordinate (B: x.c0, x.c1, y.c0, y.c1), every u64
+    limb split into its low and high 32-bit word, so that float64 holds every bit exactly."""
+    os.makedirs(d, exist_ok=True)
+    words = np.ascontiguousarray(proof, dtype="<u8").view("<u4").astype(np.float64).reshape(-1, 2 * nq)
+    for name, rows in (("a", slice(0, 2)), ("b", slice(2, 6)), ("c", slice(6, 8))):
+        np.save(os.path.join(d, f"{name}.npy"), words[rows])
 
 
 def emit(a, line):
@@ -448,12 +463,13 @@ def run_cuda(a):
             self.run_steps(z_dev.data_ptr(), ON_DEV, max(a.warmup, 3))
             first = self.step(z_dev.data_ptr(), ON_DEV).copy()
             dt, dev_ms, launches, clocks = self.timed(z_dev.data_ptr(), ON_DEV, a.steps, sampler)
+            last = proof.copy()                  # the proof of the last timed step
             lat = self.latency(z_dev.data_ptr(), ON_DEV)
             self.run_steps(z_pinned.data_ptr(), 0, 2)
             assert np.array_equal(first, proof), "resident-input and host-input proofs differ"
             dt_e, _, _, _ = self.timed(z_pinned.data_ptr(), 0, a.steps)
             tm_e = g.timings()
-            return {"proof": first, "value": units * a.steps / dt, "ms_per_step": 1e3 * dt / a.steps,
+            return {"proof": first, "last": last, "value": units * a.steps / dt, "ms_per_step": 1e3 * dt / a.steps,
                     "device_ms_per_step": statistics.mean(dev_ms), "latency_ms_single_proof": lat, "launches": int(launches),
                     "clocks": clocks, "inflight": self.inflight,
                     "e2e": {"value": units * a.steps / dt_e, "unit": "proofs/s", "h2d_bytes_per_step": int(tm_e["h2d_bytes"]),
@@ -591,6 +607,8 @@ def run_cuda(a):
             line["kernels"] = kern
         if cpu:
             line["cpu_baseline"] = cpu
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, main["last"], nq)
         emit(a, line)
     if world > 1:
         dist.barrier()

@@ -1,11 +1,13 @@
 """CPU tests of bench.py's host-side pieces (no GPU, no CUDA library): the clock sampler's timed-region window, the
 applicability rule of the committed ncu capture (`roofline.traffic`), the CPU-thread rule, and the JSON contract of the
-`--impl reference` arm on a small circuit."""
+`--impl reference` arm on a small circuit; on a GPU, the outputs --dump-outputs writes for both arms."""
 import json
 import os
 import subprocess
 import sys
 import time
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -63,10 +65,28 @@ def test_host_threads_respects_request_and_quota():
     assert 1 <= n <= (os.cpu_count() or 1)
 
 
-def test_reference_arm_line_contract_small():
+def _run_bench(args):
+    out = subprocess.run([sys.executable, "bench.py"] + args, cwd=ROOT, capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stdout + out.stderr
+    return json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
+
+
+def _load_dump(d, nq):
+    """bench.py --dump-outputs DIR -> the proof as ABI limbs (a || b || c), after checking the files' format"""
+    import numpy as np
+    parts = [np.load(os.path.join(d, f"{n}.npy")) for n in ("a", "b", "c")]
+    assert [p.shape for p in parts] == [(2, 2 * nq), (4, 2 * nq), (2, 2 * nq)] and all(p.dtype == np.float64 for p in parts)
+    words = np.concatenate([p.ravel() for p in parts])
+    assert np.all((words >= 0) & (words < 2.0 ** 32) & (words == np.floor(words)))
+    return words.astype("<u4").view("<u8")
+
+
+def test_reference_arm_line_contract_small(tmp_path):
     """`bench.py --impl reference` on a 2^10 circuit: one JSON line with the keys the driver reads, nothing of the CUDA library
-    loaded (the arm must work on a box whose libg16b200.so is absent or unloadable)."""
-    code = ("import sys, runpy; sys.argv = ['bench.py', '--impl', 'reference', '--log-n', '10', '--steps', '2', '--warmup', '1', '--cpu-threads', '2'];"
+    loaded (the arm must work on a box whose libg16b200.so is absent or unloadable); --dump-outputs writes a proof that
+    verifies for the benchmark's circuit."""
+    code = ("import sys, runpy; sys.argv = ['bench.py', '--impl', 'reference', '--log-n', '10', '--steps', '2', '--warmup', '1', '--cpu-threads', '2',"
+            f" '--dump-outputs', {str(tmp_path)!r}];"
             "runpy.run_path('bench.py', run_name='__main__');"
             "import ctypes; assert not any('libg16b200' in l for l in open('/proc/self/maps')), 'reference arm loaded the CUDA library'")
     out = subprocess.run([sys.executable, "-c", code], cwd=ROOT, capture_output=True, text=True, timeout=600)
@@ -76,6 +96,28 @@ def test_reference_arm_line_contract_small():
     assert line["metric"] == "groth16_proofs_per_sec_bls12_381_2^10" and line["steps"] == 2 and line["warmup"] == 1
     assert line["gpu_launches"] == 0 and line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["value"] == line["value"]
     assert line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] == 2
+    import types
+    import pyref as P
+    from groth16_b200 import Proof
+    from util import pk_from_abi, proof_from_abi
+    a = types.SimpleNamespace(curve="bls12_381", log_n=10, seed=1, workload="synthetic")
+    m, _, pub, _ = bench.build_workload(a)
+    pk = pk_from_abi(a.curve, bench.cpu_setup(a, m, 2))
+    nq = 6
+    limbs = _load_dump(tmp_path, nq)
+    pf = proof_from_abi(a.curve, Proof(limbs[:2 * nq], limbs[2 * nq:6 * nq], limbs[6 * nq:]))
+    assert P.verify_proof(pk.vk, P.CURVES[a.curve], pf, pub)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_cuda_equals_reference_arm(tmp_path):
+    """The CUDA arm's --dump-outputs (the last timed step) equals the reference arm's for the same arguments."""
+    import numpy as np
+    common = ["--log-n", "12", "--steps", "3", "--warmup", "1", "--cpu-threads", "4"]
+    line = _run_bench(common + ["--no-cpu-baseline", "--dump-outputs", str(tmp_path / "cuda")])
+    assert line["steps"] == 3
+    _run_bench(common + ["--impl", "reference", "--dump-outputs", str(tmp_path / "ref")])
+    assert np.array_equal(_load_dump(tmp_path / "cuda", 6), _load_dump(tmp_path / "ref", 6))
 
 
 def test_standalone_workload_generator_equals_the_library_copy():
